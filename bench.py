@@ -17,7 +17,7 @@ a trainer holding GaussianModel's tensors has to run, not a rasteriser fed pre-a
 Prints ONE JSON line on rank 0.
   value      whole-job views/s, parameters resident in HBM, one batched call per step.
   e2e        same metric through the public API with HOST buffers: pinned H2D of the raw parameter buffer + cameras, fwd+bwd,
-             D2H of loss + parameter gradients EVERY step (copies ride two copy streams, double buffered); >= 20 steps.
+             D2H of loss + parameter gradients EVERY step (copies ride two copy streams, double buffered).
   N > 1      STRONG scaling (BASELINE configs[3]): the fixed 64-camera batch is sharded over the ranks (64/N views each),
              scene broadcast once, one NCCL all-reduce of the packed gradient buffer per step inside the timed region.
              `weak_scaling` (64 views on every rank) is reported as a secondary key.
@@ -27,6 +27,10 @@ Prints ONE JSON line on rank 0.
   cuda_baseline   baseline/libb200gs_classic.so (classic-structure restatement of the reference CUDA rasteriser: per-pixel
              threads, ~10 float atomics per pixel-Gaussian pair) through the identical host path, batched and per view.
   cpu_baseline    the CPU oracle port on the host cores (bounded sample) + the reference's CPU PyTorch projection/SH paths.
+
+--dump-outputs DIR writes what the timed path returned in its last timed step as DIR/<name>.npy (float32): a fixed seed-0
+sample of the pixels and Gaussians, at most 64 MB in all.  The inputs depend on the arguments alone, so two builds run with
+the same arguments can be compared output for output.
 """
 from __future__ import annotations
 
@@ -69,7 +73,15 @@ def parse():
                     help="(internal) with --impl reference: time this many views once, plus the torch CPU paths, and print the "
                          "`cpu_baseline` object -- the GPU arm runs its CPU baseline in such a child process so that the pinned "
                          "OpenMP pool never shares a process (or a core binding) with the ranks that drive GPUs")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", default=None, metavar="DIR",
+                    help="write a fixed sample of the last timed step's outputs to DIR/<name>.npy (with --gpus N > 1: rank 0's "
+                         "views, the all-reduced gradients)")
+    args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs needs a GPU arm (--impl b200 or classic)")
+    return args
 
 
 # ------------------------------------------------------------------------------------------ clocks
@@ -311,6 +323,8 @@ class Harness:
         self.all_cams = sample_orbit_cameras(args.views, HW, HW, seed=1000, device="cpu")  # the FIXED batch, same on every rank
         self.stack = lambda cams: stack_cameras(cams, dev)
         self.stats = {}
+        self.keep_last = bool(args.dump_outputs)  # --dump-outputs: keep what step_batched returns, in self.last
+        self.last = None
 
     def camera_set(self, cams, seed):
         """device camera tensors + fixed upstream-gradient images for a list of cameras"""
@@ -332,7 +346,26 @@ class Harness:
         if self.world > 1 and allreduce:
             self.dist.all_reduce(self.flat.grad)  # the path's one exchange step: packed gradients, NCCL over NVLink
         self.stats["radii"] = r
+        if self.keep_last:
+            self.last = (c.detach(), r, d.detach(), a.detach())
         return r
+
+    def sampled_outputs(self):
+        """What the last step_batched handed its caller -- colour, depth and alpha images, radii, and the gradients of the raw
+        parameters left in flat.grad -- as float32 arrays, sampled at fixed seed-0 pixels (the same in every view) and
+        Gaussians: at most 2^20 pixel samples over all views (20 MB) and 2^23 floats of per-Gaussian rows (32 MB)."""
+        torch, R = self.torch, self.R
+        c, r, d, a = self.last
+        V, P, npix = c.shape[0], self.P, self.HW * self.HW
+        per_gaussian = V + 11 + 3 * self.K  # radii per view + xyz, scales, rotations, opacities, shs gradients
+        g = torch.Generator().manual_seed(0)
+        pix = torch.randperm(npix, generator=g)[:max(1, min(npix, (1 << 20) // V))].sort().values.to(self.dev)
+        rows = torch.randperm(P, generator=g)[:max(1, min(P, (1 << 23) // per_gaussian))].sort().values.to(self.dev)
+        out = {"color": c.flatten(2)[:, :, pix], "depth": d.flatten(2)[:, :, pix], "alpha": a.flatten(2)[:, :, pix],
+               "radii": r[:, rows].float()}
+        for name, (o, n, shape) in zip(R.PACKED_FIELDS, self.fields):
+            out["grad_" + name] = self.flat.grad.narrow(0, o, n).view(shape)[rows]
+        return {k: v.float().cpu().numpy() for k, v in out.items()}
 
     # -- the reference's unchanged calling pattern: one render() per camera, torch activations (GaussianDreamer.py:244-248)
     def step_per_view(self, cs, fused=False):
@@ -387,6 +420,20 @@ class Harness:
         bwd = sum(per(k) for k in ("blend_bwd", "preprocess_bwd"))
         return {"ms_per_step": ms / n_steps, "ms_total": ms, "fwd_ms_per_step": fwd, "bwd_ms_per_step": bwd, "stages": st, "launches": launches,
                 "steps": n_steps}
+
+
+DUMP_LIMIT_BYTES = 64 << 20
+
+
+def write_outputs(out_dir, arrays):
+    """--dump-outputs: every array as out_dir/<name>.npy; the arrays are float32 samples sized to stay under the limit."""
+    import numpy as np
+    total = sum(a.nbytes for a in arrays.values())
+    if total > DUMP_LIMIT_BYTES:
+        raise ValueError(f"--dump-outputs: {total} bytes of samples exceed {DUMP_LIMIT_BYTES}")
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, name + ".npy"), a.astype(np.float32, copy=False))
 
 
 def percentiles(xs):
@@ -540,6 +587,10 @@ def run_b200(args):
     R.profile_enable(False)
     ms_step = ms_total / args.steps
     value = args.views * args.steps / (ms_total * 1e-3)  # whole job: all ranks together render the fixed batch once per step
+    if args.dump_outputs:  # before the e2e and extra arms run other steps
+        if rank == 0:
+            write_outputs(args.dump_outputs, h.sampled_outputs())
+        h.keep_last, h.last = False, None
 
     # ---- workload statistics for the algorithmic-bytes roofline (SURVEY.md 8d; DESIGN.md "Roofline accounting")
     n_vis = int((h.stats["radii"] > 0).sum())
@@ -549,7 +600,7 @@ def run_b200(args):
     # ---- e2e through the public API with host buffers
     e2e = None
     if not args.no_e2e:
-        e2e = run_e2e(h, cs, max(args.steps, 20), W)
+        e2e = run_e2e(h, cs, args.steps, W)
 
     extras = {}
     if not args.no_extras:
@@ -756,7 +807,7 @@ def run_animation(args):
     for _ in range(W):
         step()
     torch.cuda.synchronize()
-    n = max(1, min(args.steps, 5))
+    n = args.steps
     if world > 1:
         dist.barrier()
     torch.cuda.synchronize()
@@ -773,6 +824,10 @@ def run_animation(args):
     if world > 1:
         dist.all_reduce(ms, op=dist.ReduceOp.MAX)
     ms = float(ms)
+    if args.dump_outputs and rank == 0:  # the gathered uint8 frames [F,H,W,3] at fixed seed-0 pixels, 2^22 values at most
+        npix = HW * HW
+        pix = torch.randperm(npix, generator=torch.Generator().manual_seed(0))[:max(1, min(npix, (1 << 22) // (3 * F)))]
+        write_outputs(args.dump_outputs, {"frames": out.flatten(1, 2)[:, pix.sort().values.to(dev)].float().cpu().numpy()})
     if rank == 0:
         emit({"impl": args.impl, "metric": "animation frames/sec @1024^2, sample.ply (BASELINE config 5)", "value": F * n / (ms * 1e-3), "unit": "frames/s",
               "n_gpus": world, "steps": n, "warmup": W, "ms_per_step": ms / n, "higher_is_better": True, "scaling": "strong", "vs_baseline": None,

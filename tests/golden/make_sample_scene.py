@@ -7,8 +7,8 @@ the real anisotropy / opacity distribution.  Run in the authoring container only
 Stored: `data` float32 [N,14] = the 14 non-constant PLY columns (x y z f_dc_0..2 opacity scale_0..2 rot_0..3) in file
 order, `columns` = their names.  The three normal columns of the file are identically 0 (checked) and not stored.
 humangaussian_b200.scene.sample_ply_scene() rebuilds the raw GaussianParams exactly as the reference's load_ply does
-(gaussiansplatting/scene/gaussian_model.py:225-266); tests/test_oracle_golden.py checks the rebuilt columns against a
-re-read of the PLY when /root/reference is present.
+(gaussiansplatting/scene/gaussian_model.py:225-266); tests/test_ply_codec.py checks the rebuilt tensors against what the
+PLY codec reads from the file itself (recorded by make_sample_ply_check.py).
 """
 import os
 import sys

@@ -23,6 +23,14 @@ def test_reference_arm_prints_exactly_one_json_line_with_the_contract_keys():
     assert d["gpu_launches"] == 0 and "workload" in d["config"]
 
 
+def test_arguments_that_cannot_be_honoured_are_refused():
+    """No timed steps, or an output dump from the CPU arm (which returns no GPU outputs), is an argument error."""
+    for extra in (["--steps", "0"], ["--impl", "reference", "--dump-outputs", "unused"]):
+        out = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py")] + extra, capture_output=True, text=True, timeout=600, cwd=ROOT)
+        assert out.returncode == 2 and "error" in out.stderr, (extra, out.stderr[-2000:])
+        assert not os.path.exists(os.path.join(ROOT, "unused"))
+
+
 def test_clock_sampler_degrades_without_nvidia_smi(monkeypatch):
     sys.path.insert(0, ROOT)
     import bench

@@ -1,6 +1,7 @@
 """CPU: the PLY codec (humangaussian_b200/scene.py) against fixtures produced by RUNNING the reference's own save_ply /
 load_ply (tests/golden/make_golden_ply.py): gaussiansplatting/scene/gaussian_model.py:187-266 (training convention) and
 gs_renderer.py:525-610 (animation convention: y/z swap, quaternion 2<->3 swap, component-0 negation, file-order columns)."""
+import hashlib
 import os
 
 import numpy as np
@@ -81,19 +82,23 @@ def test_reader_rejects_what_it_cannot_parse(tmp_path):
         params_from_ply(_file(tmp_path, "deg2_file"), sh_degree=1)  # wrong number of f_rest columns for the degree
 
 
-def test_sample_scene_pack_matches_the_ply_when_the_reference_is_present():
-    """tests/golden/sample_ply_full.npz is content/sample.ply repacked: same tensors as loading the PLY itself."""
+def test_sample_scene_pack_matches_the_ply():
+    """tests/golden/sample_ply_full.npz is content/sample.ply repacked: same tensors as loading the PLY itself, as recorded
+    from the reference's file by tests/golden/make_sample_ply_check.py (bit-exact digests of every tensor, plus sampled rows)."""
     p = sample_ply_scene()
     assert p.P == 531327 and p.features_rest.shape == (531327, 0, 3)
     op = torch.sigmoid(p.opacity)
     assert abs(float(op.mean()) - 0.103) < 2e-3                      # SURVEY.md 8c's measured statistics of the file
     assert abs(float(torch.exp(p.scaling).median()) - 0.0028) < 2e-4
-    ref = "/root/reference/content/sample.ply"
-    if os.path.exists(ref):
-        for conv in ("training", "animation"):
-            q = params_from_ply(ref, 0, conv)
-            r = sample_ply_scene(convention=conv)
-            for k in KEYS:
-                assert torch.equal(getattr(q, k), getattr(r, k)), (conv, k)
+    ply = np.load(os.path.join(ROOT, "tests", "golden", "sample_ply_check.npz"))
+    rows = torch.from_numpy(ply["row_index"])
+    for conv in ("training", "animation"):
+        r = sample_ply_scene(convention=conv)
+        for k in KEYS:
+            t = getattr(r, k)
+            assert list(t.shape) == ply[f"{conv}_{k}_shape"].tolist(), (conv, k)
+            assert np.array_equal(t[rows].numpy(), ply[f"{conv}_{k}_rows"]), (conv, k)
+            digest = hashlib.sha256(np.ascontiguousarray(t.numpy(), dtype=np.float32).tobytes()).hexdigest()
+            assert digest == str(ply[f"{conv}_{k}_sha256"]), (conv, k)
     s = sample_ply_scene(300000, 3)
     assert s.P == 300000 and s.features_rest.shape == (300000, 15, 3) and abs(float(s.features_rest.std()) - 0.1) < 1e-3
